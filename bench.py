@@ -6,9 +6,12 @@
 
 One JSON line on stdout (rank 0).  A "step" is one full training step of Trainer (sampled batch of 1024 interactions +
 augmented edges: forward, 8 BPR/prune heads, backward, dense AdamW).
-  value         whole-job interactions/s with the batch indices already resident in HBM: blocks of EXACTLY --steps steps between
-                CUDA events (synchronize on both sides), repeated until >= --min-seconds of device time; the MEDIAN block is reported
+  value         whole-job interactions/s with the batch indices already resident in HBM: EXACTLY --steps consecutive steps after
+                --warmup (at least 3) untimed ones, between two CUDA events (synchronize on both sides); an event after every step gives
+                the per-step min / max.  Before the timed window the same steps are replayed for --min-seconds of device time so that
+                clocks and caches are in steady state; the parameter and optimizer updates of those replays are undone
   e2e           the same through Trainer's public API: host sampler -> pinned H2D of the index batch -> step -> D2H of the loss, every step
+                (blocks of --steps steps, repeated until >= --min-seconds / 2 of device time; the median block is reported)
   roofline      the dominant kernel family of the step: algorithmic bytes / CUDA-event time vs MEASURED_PEAKS.json
   cpu_baseline  the oracle port (oracle/llmrec_oracle.py, torch CPU) on a bounded sample of the same workload
   gpu_torch_baseline  the same oracle ops with every tensor on cuda:0 (torch.sparse.mm / F.linear / AdamW = cuSPARSE / cuBLAS / ATen):
@@ -18,6 +21,10 @@ augmented edges: forward, 8 BPR/prune heads, backward, dense AdamW).
   configs       the other BASELINE.json configurations measured in the same call: movielens d=128 L=3 (configs[2]); the 10M x 1M synthetic on
                 this one GPU (= `scaling_base`, the strong-scaling base of the N > 1 lines, configs[3]) with its 1M-item eval leg (configs[4])
 Features (704 MB) exceed the 126 MB L2, so consecutive steps cannot be served from cache ("inputs larger than L2").
+
+--dump-outputs DIR writes what the last timed step left to its caller, one float32 array per file: DIR/loss.npy and DIR/<parameter
+name>.npy for every parameter after that step's AdamW update.  Dataset, initialisation and batches are seeded, so two builds run with
+the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -27,6 +34,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -51,7 +59,8 @@ def workload_string(name):
 def ensure_dataset(name):
     from llmrec_b200.synth import make_dataset
     ds, nu, ni, ne, dims, _, _ = WORKLOADS[name]
-    root = os.path.join(os.environ.get("LLMREC_BENCH_DIR", "/tmp/llmrec_bench"), f"{name}_seed0") + "/"
+    base = os.environ.get("LLMREC_BENCH_DIR") or os.path.join(tempfile.gettempdir(), f"llmrec_bench_{os.getuid()}")
+    root = os.path.join(base, f"{name}_seed0") + "/"
     marker = os.path.join(root, ".complete")
     if not os.path.exists(marker):
         os.makedirs(root, exist_ok=True)
@@ -122,8 +131,8 @@ def make_trainer(workload, a, extra=()):
     return tr, gen, args
 
 
-def time_steps(tr, a, K, W, min_seconds, max_blocks):
-    """-> dict(ms_per_step median, min, max, blocks, value, launches) for the device-resident leg of Trainer `tr`."""
+def time_steps(tr, a, K, W, min_seconds, max_blocks, dump_dir=None):
+    """-> dict(ms, value, ms_min, ms_max, launches) for EXACTLY K timed steps of the device-resident leg of Trainer `tr`."""
     import torch
     from llmrec_b200 import ops
     hp = tr.hot
@@ -135,30 +144,54 @@ def time_steps(tr, a, K, W, min_seconds, max_blocks):
     step = hp.train_step_graphed if a.graph else hp.train_step
     for i in range(W):
         step(*dev_batches[i])
-    torch.cuda.synchronize()
+    snap = hp._snapshot_state()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    blocks, spent = [], 0.0
-    l0 = ops.STATS["launches"]
-    while True:
-        torch.cuda.synchronize()
+    spent, blocks = 0.0, 0
+    while spent < 1e3 * min_seconds and blocks < max_blocks:
         e0.record()
         for i in range(W, W + K):
             step(*dev_batches[i])
         e1.record()
         torch.cuda.synchronize()
-        ms = e0.elapsed_time(e1)
-        blocks.append(ms); spent += ms
-        if spent >= 1e3 * min_seconds or len(blocks) >= max_blocks:
-            break
-    launches = (ops.STATS["launches"] - l0) // len(blocks)
+        spent += e0.elapsed_time(e1); blocks += 1
+    hp._restore_state(snap)
+    del snap
+    torch.cuda.synchronize()
+    ev = [torch.cuda.Event(enable_timing=True) for _ in range(K + 1)]
+    l0 = ops.STATS["launches"]
+    ev[0].record()
+    for i in range(K):
+        step(*dev_batches[W + i])
+        ev[i + 1].record()
+    torch.cuda.synchronize()
+    launches = ops.STATS["launches"] - l0
+    if dump_dir is not None:
+        dump_outputs(hp, dump_dir)
+    per_step = [ev[i].elapsed_time(ev[i + 1]) for i in range(K)]
     if a.graph:      # kernels per replayed step = launches of one eager step
         l1 = ops.STATS["launches"]
         snap = hp._snapshot_state(); hp.train_step(*dev_batches[0]); hp._restore_state(snap)
         launches = (ops.STATS["launches"] - l1) * K
     n_inter = sum(len(b[0]) for b in batches[W:])
-    ms = _median(blocks)
-    return {"ms": ms, "value": n_inter / (ms / 1e3), "blocks": len(blocks), "ms_min": min(blocks), "ms_max": max(blocks), "launches": launches,
+    ms = ev[0].elapsed_time(ev[K])
+    return {"ms": ms, "value": n_inter / (ms / 1e3), "ms_min": min(per_step), "ms_max": max(per_step), "launches": launches,
             "dev_batches": dev_batches}
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(hp, out_dir):
+    """DIR/loss.npy and DIR/<parameter name>.npy (float32) as the last step left them (about 9 MB at netflix shape, 14 MB at movielens shape)."""
+    import numpy as np
+    arrays = {"loss": hp.loss.detach().float().cpu().numpy()}
+    arrays.update({k: v.detach().float().cpu().numpy() for k, v in hp.p.items()})
+    total = sum(v.nbytes for v in arrays.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
 
 
 def time_e2e(tr, K, min_seconds, max_blocks):
@@ -238,16 +271,16 @@ def eval_leg(tr, gen, ni, shots=5):
             "recall@20": float(res["recall"][1]), "ndcg@20": float(res["ndcg"][1]), "includes": "forward + scoring + top-50 + metrics, host buffers"}
 
 
-def run_workload(name, a, K, W, min_seconds, with_families=True, hoist=False, extra=()):
-    """One single-GPU configuration: device-resident leg, e2e leg, family roofline, eval leg."""
+def run_workload(name, a, K, W, min_seconds, with_families=True, hoist=False, extra=(), dump_dir=None):
+    """One single-GPU configuration: device-resident leg (its outputs written to `dump_dir` if given), e2e leg, family roofline, eval leg."""
     import torch
     from llmrec_b200.roofline import peaks, step_bytes
     tr, gen, args = make_trainer(name, a, extra=(["--hoist_side", "1"] if hoist else []) + list(extra))
     ds, nu, ni, ne, dims, embed, wsize = WORKLOADS[name]
-    t = time_steps(tr, a, K, W, min_seconds, a.max_blocks)
+    t = time_steps(tr, a, K, W, min_seconds, a.max_blocks, dump_dir)
     e2e = time_e2e(tr, K, min_seconds / 2, a.max_blocks)
     out = {"workload": workload_string(name), "ms_per_step": round(t["ms"] / K, 4), "value": round(t["value"], 1), "unit": "interactions/s",
-           "blocks": t["blocks"], "ms_per_step_min": round(t["ms_min"] / K, 4), "ms_per_step_max": round(t["ms_max"] / K, 4),
+           "ms_per_step_min": round(t["ms_min"], 4), "ms_per_step_max": round(t["ms_max"], 4),
            "e2e": e2e, "gpu_launches": t["launches"], "train_edges": int(gen.n_train)}
     if with_families and not hoist:
         fam = family_times(tr, t["dev_batches"][0])
@@ -386,7 +419,7 @@ def run_ours(a):
     K, W = a.steps, max(a.warmup, 3)
     ds, nu, ni, ne, dims, embed, wsize = WORKLOADS[a.workload]
     clocks = ClockSampler(0); clocks.start()      # samples clocks / throttle reasons across the value and e2e legs
-    main, tr, gen = run_workload(a.workload, a, K, W, a.min_seconds)
+    main, tr, gen = run_workload(a.workload, a, K, W, a.min_seconds, dump_dir=a.dump_outputs)
     clk = clocks.finish()
     out = {"metric": "train_interactions_per_sec", "value": main["value"], "unit": "interactions/s", "n_gpus": 1, "steps": K, "warmup": W,
            "ms_per_step": main["ms_per_step"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32",
@@ -394,7 +427,7 @@ def run_ours(a):
            "config": {"workload": workload_string(a.workload), "train_edges": main["train_edges"],
                       "interactions_counted": "sum(len(users)) incl. augmented edges", "l2": "inputs larger than L2 (704 MB of features per step)",
                       "proj_mode": a.proj_mode, "host_sampler": a.host_sampler, "cuda_graph": bool(a.graph),
-                      "timing": f"median of {main['blocks']} blocks of {K} steps (>= {a.min_seconds} s of device time)",
+                      "timing": f"{K} consecutive steps between CUDA events after {W} untimed ones",
                       "ms_per_step_min": main["ms_per_step_min"], "ms_per_step_max": main["ms_per_step_max"]},
            "e2e": main["e2e"], "gpu_launches": main["gpu_launches"], "clocks": clk, "roofline": main["roofline"], "eval": main["eval"]}
     del tr
@@ -477,11 +510,11 @@ def run_reference(a):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed training steps (N=1: exactly this many; the e2e leg times blocks of this many)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="netflix", choices=list(WORKLOADS) + ["synthetic"])
-    ap.add_argument("--min-seconds", dest="min_seconds", type=float, default=2.0, help="repeat the K-step block until this much device time; the median block is reported")
+    ap.add_argument("--min-seconds", dest="min_seconds", type=float, default=2.0, help="N=1: untimed replays of the K timed steps before they are timed, and the e2e leg's repeated K-step blocks; N>1: repeat the K-step block until this much device time, the median block is reported")
     ap.add_argument("--max-blocks", dest="max_blocks", type=int, default=400)
     ap.add_argument("--pieces", type=int, default=1, help="N>1: item-row pieces of the exchange SpMMs (all-reduce of piece k overlaps SpMM of piece k+1)")
     ap.add_argument("--item-sharded", dest="item_sharded", type=int, default=0, help="N>1: reduce-scatter / row-local work / all-gather form of the item-side exchanges, AdamW of the item table sharded by item")
@@ -497,7 +530,11 @@ def main():
     ap.add_argument("--graph", type=int, default=1)
     ap.add_argument("--cpu-steps", dest="cpu_steps", type=int, default=24)
     ap.add_argument("--cpu-eval-users", dest="cpu_eval_users", type=int, default=1500)
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR", default=None,
+                    help="N=1: write the loss and the parameters after the last timed step to DIR/<name>.npy (float32)")
     a = ap.parse_args()
+    if a.dump_outputs is not None and (a.impl != "ours" or a.gpus > 1 or a.workload == "synthetic"):
+        ap.error("--dump-outputs covers the single-GPU CUDA path (--impl ours --gpus 1, workload netflix or movielens)")
     if a.workload == "synthetic" and a.impl == "reference":
         a.workload = "netflix"
     out = run_reference(a) if a.impl == "reference" else run_ours(a)

@@ -214,7 +214,7 @@ def run_sharded(a, dev=None):
            "e2e": {"value": round(B * K / (ms2 / 1e3), 1), "unit": "interactions/s", "h2d_bytes_per_step": 3 * 4 * B, "d2h_bytes_per_step": 4,
                    "ms_per_step": round(ms2 / K, 4)},
            "gpu_launches": launches, "same_workload_1gpu": base, "scaling_base": base,
-           "roofline": {"kernel": "spmm gather (item-side product R_r^T . U, one rank)", "bound": "hbm", "achieved": round(alg / (t_spmm * 1e-3) / 1e9, 1),
+           "roofline": {"kernel": "spmm gather (item-side product R_r^T . U, one rank)", "bound": "hbm", "achieved": round(alg / (t_spmm * 1e-3) / 1e9, 4),
                         "peak": hbm, "unit": "GB/s", "frac": round(alg / (t_spmm * 1e-3) / 1e9 / hbm, 4), "traffic": None, "peak_source": src,
                         "alg_bytes": alg, "ms": round(t_spmm, 4), "gather_bound_gbs": round(gather / (t_spmm * 1e-3) / 1e9, 1),
                         "note": "achieved uses compulsory bytes (every operand once); gather_bound_gbs counts one row read per non-zero"},

@@ -24,7 +24,7 @@ def test_sharded_demand_world1_equals_engine():
 
 def test_sharded_demand_world2_equals_engine():
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     r = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2", "--master-addr", "127.0.0.1",
                         "--master-port", "29521", os.path.join(HERE, "dist_gpu_check.py")], capture_output=True, text=True, timeout=600,
                        env=dict(os.environ, LLMREC_DIST_DEMAND="1"))
@@ -33,7 +33,7 @@ def test_sharded_demand_world2_equals_engine():
 
 def test_sharded_world2_equals_engine():
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     r = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2", "--master-addr", "127.0.0.1",
                         "--master-port", "29517", os.path.join(HERE, "dist_gpu_check.py")], capture_output=True, text=True, timeout=600)
     assert "DIST_CHECK_OK" in r.stdout, r.stdout[-2000:] + r.stderr[-2000:]
@@ -43,7 +43,7 @@ def test_sharded_world2_equals_engine():
 def test_item_sharded_exchange_world2_equals_engine():
     """dist.ShardedHotPath(item_sharded=True): reduce-scatter / row-local / all-gather form == single-GPU engine."""
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     here = HERE
     env = dict(os.environ, LLMREC_DIST_ITEM_SHARDED="1")
     r = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2", "--master-addr", "127.0.0.1",
